@@ -10,6 +10,7 @@ so that the CPU test-suite (and the GPU box) can pin oracle/ and dalm_b200's hos
   preprocess.json reference batch builders (e2e + retriever-only) on synthetic rows with the fixture tokenizers
   eval_helpers.json reference dalm/eval/utils.py helpers (precision/recall, result aggregation, unique-passage filter,
                   tokenisation, neighbour formatting over a fixed (labels, distances) answer) — hnswlib itself is stubbed
+  reference_spot_checks.json  reference compute_marginalized_loss_from_logits on a fresh seed, and eval-helper spot checks
 """
 from __future__ import annotations
 
@@ -144,6 +145,38 @@ def gen_eval_helpers(ref):
         json.dump(out, f)
 
 
+def spot_check_marginal_inputs():
+    """inputs of the fresh-seed marginalized-loss check (tests/test_oracle_golden.py), separate from loss_cases()"""
+    g = torch.Generator().manual_seed(123)
+    B, L, V, D = 6, 10, 31, 24
+    q = torch.nn.functional.normalize(torch.randn(B, D, generator=g), dim=1)
+    p = torch.nn.functional.normalize(torch.randn(B, D, generator=g), dim=1)
+    lg = torch.randn(B, L, V, generator=g); ids = torch.randint(0, V, (B, L), generator=g)
+    mask = torch.ones(B, L, dtype=torch.int64); mask[2, :4] = 0; mask[4, 7:] = 0
+    ql = torch.tensor([1, 2, 9, 10, 12, 5])
+    return q, p, lg, ids, mask, ql
+
+
+SPOT_PRECISION_RECALL = [(["a", "b"], ["b"]), (["k"] * 4, ["k"]), (["m", "n", "o"], ["z"])]
+SPOT_EVAL_RESULTS = (5, [0.1] * 5, [1, 0, 1, 1, 0], 3)
+
+
+def gen_spot_checks(ref):
+    """the reference's answers for the fresh-seed loss check and the eval-helper spot checks"""
+    q, p, lg, ids, mask, ql = spot_check_marginal_inputs()
+    S = ref.train_utils.get_cosine_sim(q, p, 100)
+    lm = ref.train_utils.compute_marginalized_loss_from_logits(lg, ids, mask, S, ql)
+    eu = ref.eval_utils
+    res = eu.calc_eval_results(*SPOT_EVAL_RESULTS)
+    out = {"marginalized_loss": {"dtype": str(lm.dtype).replace("torch.", ""), "value": lm.item()},
+           "precision_recall": [{"retrieved": r, "correct": c, "out": list(eu.calculate_precision_recall(r, c))}
+                                for r, c in SPOT_PRECISION_RECALL],
+           "calc_eval_results": {"args": list(SPOT_EVAL_RESULTS),
+                                 "out": res.model_dump() if hasattr(res, "model_dump") else res.dict()}}
+    with open(os.path.join(GOLD, "reference_spot_checks.json"), "w") as f:
+        json.dump(out, f, indent=1)
+
+
 def main():
     from oracle import ref_import
 
@@ -153,6 +186,7 @@ def main():
     gen_pooling(ref)
     gen_preprocess(ref)
     gen_eval_helpers(ref)
+    gen_spot_checks(ref)
     print("golden fixtures written to", GOLD)
 
 

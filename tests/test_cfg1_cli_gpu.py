@@ -17,10 +17,9 @@ TOY = os.path.join(ROOT, "tests", "golden", "ref_toy_data_train.csv")
 
 
 def test_toy_fixture_is_the_reference_file():
-    """when the reference tree is present (build container) the committed fixture must be byte-identical to it"""
-    ref = "/root/reference/dalm/datasets/toy_data_train.csv"
-    if os.path.exists(ref):
-        assert open(ref, "rb").read() == open(TOY, "rb").read()
+    """the committed fixture is byte-identical to the reference's dalm/datasets/toy_data_train.csv (its SHA-256)"""
+    import hashlib
+    assert hashlib.sha256(open(TOY, "rb").read()).hexdigest() == "783d2a65fdccc11c5f88bf351469af579547c48296c0c8544f7b9d9a97cba477"
     import csv
     rows = list(csv.DictReader(open(TOY)))
     assert {"Question", "Abstract", "Answer"} <= set(rows[0]) and len(rows) >= 10
